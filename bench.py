@@ -151,6 +151,23 @@ def by_id(torch, state, ids_wanted):
     return tuple(state[k][pos].cpu().numpy() for k in ('lon', 'lat', 'z'))
 
 
+DUMP_PARTICLES = 2_000_000     # lon, lat (float64) and z (float32) of this many elements over all ranks: 40 MB
+
+
+def dump_outputs(out_dir, torch, state, rank, world):
+    """What the timed steps computed: the final lon / lat / z a caller of the step receives, in element order, as
+    out_dir/<name>.npy (a rank suffix per process when there are several).  Above DUMP_PARTICLES / world elements a fixed,
+    seeded sample of element ids is written, the same in every run."""
+    n, m = state['ids'].numel(), DUMP_PARTICLES // world
+    ids = np.arange(n)
+    if n > m:
+        ids = np.sort(np.random.default_rng(7).choice(n, size=m, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = '_rank%d' % rank if world > 1 else ''
+    for name, a in zip(('lon', 'lat', 'z'), by_id(torch, state, ids)):
+        np.save(os.path.join(out_dir, name + suffix + '.npy'), a)
+
+
 def parity_of_timed_run(eng, torch, st, snap, par_steps, step, args):
     """(a) the last `par_steps` TIMED steps: a subsample of the snapshot taken inside the timed region is advanced by the CPU
     oracle (oracle/advect_port.py, bit-identical to the reference on the committed fixtures) and compared with the positions
@@ -327,7 +344,7 @@ def run_b200(args):
     dev = eng.device
     n = args.particles
     grid = syn.GridSpec()
-    n_times = syn.n_slabs_for(args.warmup + 3 * args.steps + 4, DT) + PERIOD        # (room for two repeats of the timed region)
+    n_times = syn.n_slabs_for(args.warmup + 3 * args.steps + 4, DT) + PERIOD        # (room for the steps after the timed region)
     times = syn.slab_times(n_times)
 
     # Forcing: rank 0 "reads" the slabs (builds them on the host, keeps them pinned and resident); in a distributed run the other
@@ -448,46 +465,31 @@ def run_b200(args):
 
     def snapshot():
         return {k: st[k].clone() for k in ('lon', 'lat', 'z', 'ids')}, st['t'], st['k']
-    # The timed region is K steps of ~1 ms.  A single stall of the box (observed once in this round: 78 ms of idle device time
-    # between two steps of a 20 ms region, nothing of the kind in the runs before and after) would turn the number into a
-    # measurement of that stall.  The region is therefore checked: the device time between the steps' own events (end of step j
-    # to start of step j + 1) is summed, and if more than 20 % of the region was such idle time the K steps are timed again on
-    # the continuing simulation (at most twice; every attempt is K complete steps and is listed in `timed_region_attempts`).
-    attempts = []
-    for attempt in range(3):
-        del step_events[:]
-        del host_us[:]
-        snap = snapshot() if snap_at == 0 and not args.no_parity else None
-        wall0 = _dt.now()
-        e0.record()
-        for j in range(args.steps):
-            if j == snap_at and j > 0 and not args.no_parity:
-                snap = snapshot()
-            step(record=True)
-        e1.record()
-        barrier()
-        wall1 = _dt.now()
-        ms_total = e0.elapsed_time(e1)
-        busy = float(sum(a.elapsed_time(b) for a, b in step_events))
-        idle = ms_total - busy
-        retry = idle > 0.2 * ms_total
-        if world > 1:                   # every rank must take the same decision
-            flag = torch.tensor([1.0 if retry else 0.0], device=dev)
-            dist.all_reduce(flag, op=dist.ReduceOp.MAX)
-            retry = bool(flag.item() > 0)
-        attempts.append({'ms_total': ms_total, 'ms_in_steps': busy, 'ms_idle_between_steps': idle, 'repeated': bool(retry and attempt < 2)})
-        if not retry or attempt == 2:
-            break
-        l0 = eng.launches()
-        bc0 = eng.dist.slabs_broadcast if eng.dist is not None else 0
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        barrier()
+    # Exactly K timed steps.  The device time between the steps' own events (end of step j to start of step j + 1) is reported
+    # beside the total: a stall of the shared box shows there rather than hiding in the step times.
+    del step_events[:]
+    del host_us[:]
+    snap = snapshot() if snap_at == 0 and not args.no_parity else None
+    wall0 = _dt.now()
+    e0.record()
+    for j in range(args.steps):
+        if j == snap_at and j > 0 and not args.no_parity:
+            snap = snapshot()
+        step(record=True)
+    e1.record()
+    barrier()
+    wall1 = _dt.now()
+    ms_total = e0.elapsed_time(e1)
+    busy = float(sum(a.elapsed_time(b) for a, b in step_events))
+    timed_region = {'ms_total': ms_total, 'ms_in_steps': busy, 'ms_idle_between_steps': ms_total - busy}
     gc.enable()
     launches = eng.launches() - l0
     slabs_bcast = (eng.dist.slabs_broadcast - bc0) if eng.dist is not None else 0
     loop_kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in step_events]))   # includes slab upload / pair packing
     clocks = sampler.stop(wall0, wall1) if sampler else None
     per_step = np.array([a.elapsed_time(b) for a, b in step_events])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, torch, st, rank, world)
     if os.environ.get('OD_BENCH_DEBUG'):          # per-step device times and the gaps between steps, every rank
         gaps = [step_events[k][1].elapsed_time(step_events[k + 1][0]) for k in range(len(step_events) - 1)]
         os.makedirs(os.path.join(ROOT, 'gpurun_out'), exist_ok=True)
@@ -720,7 +722,7 @@ def run_b200(args):
                                   if world > 1 else 'single GPU',
                    'l2': 'inputs larger than L2 (state %.0f MB + forcing %.0f MB per step)' % (n * 20 / 1e6, field_bytes / 1e6)},
         'clocks': clocks,
-        'timed_region_attempts': attempts,
+        'timed_region': timed_region,
         'comm': {'slab_broadcasts_in_timed_region': slabs_bcast, 'broadcast': bcast, 'numa': numa,
                  'slab_broadcast_communicator_max_ctas': getattr(eng.dist, 'bcast_ctas', None)} if world > 1 else {'numa': numa},
         'e2e': {'value': e2e_value, 'unit': 'particle-steps/s', 'h2d_bytes_per_step': n * 20, 'd2h_bytes_per_step': n * 20,
@@ -784,7 +786,11 @@ def main():
     ap.add_argument('--api-steps', type=int, default=120, help='steps of the OceanDrift.run() leg')
     ap.add_argument('--cfg4-particles', type=int, default=5_000_000)
     ap.add_argument('--cfg5-particles', type=int, default=20_000_000)
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the positions the timed steps computed to DIR/<name>.npy '
+                                                          '(--impl b200 only: the reference arm has no such steps)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to --impl b200 only')
     if args.warmup < 3 and args.impl == 'b200':
         args.warmup = 3
     if args.impl == 'reference':

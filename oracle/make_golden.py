@@ -193,15 +193,12 @@ def run_leeway_case(name, g, n, steps, dt, object_type=1, seed=0, capsizing=None
     print('wrote', path, 'max |dlon|', np.abs(o.elements.lon - lon).max(), 'jibed', int((o.elements.orientation != np.r_[:n] % 2).sum()))
 
 
-def run_dateline_case(name, field, seeds_lon, seeds_lat, steps, dt, scheme='euler', wdf=0.1):
-    """The reference's tests/readers/test_interpolation.py:43-148 (test_dateline) with in-memory readers: a current
-    reader on lon 0..359 (global, 0-360 convention) and a wind reader on lon -180..179 (global, -180-180 convention),
-    lat -88..88, daily slabs.  field='piecewise' are the test's own fields (u = +1 east of 0, -1 west; wind v = +1 on
-    the western half of its grid, -1 on the eastern); 'smooth' varies with lon / lat so that the seam cells matter."""
+def dateline_fields(field):
+    """The readers' axes and fields of the dateline cases: latitude, the current's and the wind's longitudes, u, v, x_wind, y_wind.
+    Pure NumPy: the 'smooth' fixtures do not store their fields, the tests rebuild them here."""
     lat = np.arange(-88, 89).astype(np.float32)
     lon_c = np.arange(0, 360).astype(np.float32)
     lon_w = np.arange(-180, 180).astype(np.float32)
-    times = syn.slab_times(3, 86400)
     ny = len(lat)
     if field == 'piecewise':
         u = np.zeros((3, ny, 360), np.float32); v = np.zeros_like(u)
@@ -217,6 +214,16 @@ def run_dateline_case(name, field, seeds_lon, seeds_lat, steps, dt, scheme='eule
         v = np.stack([(0.3 * np.sin(3 * lo_c) * np.cos(la) * (1 + 0.1 * k)) for k in range(3)]).astype(np.float32)
         xw = np.stack([(8.0 * np.cos(lo_w + 0.2 * k) * np.cos(la)) for k in range(3)]).astype(np.float32)
         yw = np.stack([(5.0 * np.sin(2 * lo_w) + 1.0 * k) for k in range(3)]).astype(np.float32)
+    return lat, lon_c, lon_w, u, v, xw, yw
+
+
+def run_dateline_case(name, field, seeds_lon, seeds_lat, steps, dt, scheme='euler', wdf=0.1):
+    """The reference's tests/readers/test_interpolation.py:43-148 (test_dateline) with in-memory readers: a current
+    reader on lon 0..359 (global, 0-360 convention) and a wind reader on lon -180..179 (global, -180-180 convention),
+    lat -88..88, daily slabs.  field='piecewise' are the test's own fields (u = +1 east of 0, -1 west; wind v = +1 on
+    the western half of its grid, -1 on the eastern); 'smooth' varies with lon / lat so that the seam cells matter."""
+    lat, lon_c, lon_w, u, v, xw, yw = dateline_fields(field)
+    times = syn.slab_times(3, 86400)
     lon0 = np.asarray(seeds_lon, dtype=np.float32)
     lat0 = np.asarray(seeds_lat, dtype=np.float32)
     n = len(lon0)
@@ -231,8 +238,9 @@ def run_dateline_case(name, field, seeds_lon, seeds_lat, steps, dt, scheme='eule
                 wind_drift_depth=None, start_offset_s=0, start_index=None, slab_step_s=86400, cdf_is_array=False,
                 mixing=False, dt_mix=60.0, stokes=None, noise=None, wdf=wdf, field=field)
     path = os.path.join(OUT, 'ref_%s.npz' % name)
-    np.savez_compressed(path, meta=json.dumps(meta), grid_lon=lon_c, grid_lat=lat, grid_z=np.zeros(0), u=u, v=v,
-                        x_wind=xw, y_wind=yw, wind_lon=lon_w, wind_lat=lat, lon0=lon0, lat0=lat0, z0=z0,
+    fields = dict(u=u, v=v, x_wind=xw, y_wind=yw) if field == 'piecewise' else {}       # (the smooth ones would exceed 1 MB)
+    np.savez_compressed(path, meta=json.dumps(meta), grid_lon=lon_c, grid_lat=lat, grid_z=np.zeros(0), **fields,
+                        wind_lon=lon_w, wind_lat=lat, lon0=lon0, lat0=lat0, z0=z0,
                         lon=np.asarray(o.elements.lon, dtype=np.float64), lat=np.asarray(o.elements.lat, dtype=np.float64),
                         z=np.asarray(o.elements.z))
     print('wrote', path, 'first four', np.asarray(o.elements.lon)[:4], np.asarray(o.elements.lat)[:4])
@@ -307,6 +315,11 @@ def gyre_cases():
 # The forcing is syn.* on the full 512 x 512 x 50 grid: it is regenerated by the tests from the same formulas, so the fixtures hold
 # only the configuration and the reference's final state (seeds: syn.particle_cloud(n, seed)).
 BIG_N = 100_000
+BIG_SAMPLE = 30_000        # elements whose final state is stored: a fixed, seeded sample of the BIG_N that run (keeps a fixture < 1 MB)
+
+
+def big_sample_ids():
+    return np.sort(np.random.default_rng(2024).choice(BIG_N, size=BIG_SAMPLE, replace=False)).astype(np.int32)
 
 
 def big_fields(kind, n_slabs):
@@ -355,14 +368,15 @@ def run_big_case(kind):
     o = refrun.run_oceandrift(readers, lon, lat, z if c['model'] != 'Leeway' else 0, start, c['dt'], c['steps'], config=c['config'],
                               seed_kwargs=kw, model=c['model'], seed=0)
     assert len(o.elements.lon) == BIG_N, 'reference deactivated particles in %s' % kind
-    out = dict(meta=json.dumps(dict(kind=kind, n=BIG_N, n_slabs=n_slabs, **{k: v for k, v in c.items()})),
-               lon=np.asarray(o.elements.lon, dtype=np.float64), lat=np.asarray(o.elements.lat, dtype=np.float64))
+    ids = big_sample_ids()
+    out = dict(meta=json.dumps(dict(kind=kind, n=BIG_N, n_slabs=n_slabs, **{k: v for k, v in c.items()})), ids=ids,
+               lon=np.asarray(o.elements.lon, dtype=np.float64)[ids], lat=np.asarray(o.elements.lat, dtype=np.float64)[ids])
     if c['model'] == 'Leeway':
-        out['orientation'] = np.asarray(o.elements.orientation).astype(np.int8)
+        out['orientation'] = np.asarray(o.elements.orientation).astype(np.int8)[ids]
     else:
-        out['z'] = np.asarray(o.elements.z)
+        out['z'] = np.asarray(o.elements.z)[ids]
     np.savez_compressed(os.path.join(OUT, 'ref_big_%s.npz' % kind), **out)
-    print('wrote ref_big_%s' % kind, 'max |dlon|', np.abs(out['lon'] - lon).max(), 'z dtype', out.get('z', np.zeros(0)).dtype)
+    print('wrote ref_big_%s' % kind, 'max |dlon|', np.abs(out['lon'] - lon[ids]).max(), 'z dtype', out.get('z', np.zeros(0)).dtype)
 
 
 def main():

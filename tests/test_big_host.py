@@ -41,11 +41,12 @@ def test_benchmarked_configuration_on_the_host_build(kind, sort, ztol, host_engi
 
 
 def test_port_matches_reference_on_cfg2_subsample():
-    """oracle/advect_port.py (the CPU baseline of bench.py) on the first 4000 particles of cfg 2."""
+    """oracle/advect_port.py (the CPU baseline of bench.py) on the first 4000 stored particles of cfg 2."""
     from oracle import advect_port as ap
     c = _case('cfg2')
     m = 4000
+    s = c.ref['ids'][:m]
     f = c.fields['current']
     rd = ap.GridReader(c.grid.lon, c.grid.lat, c.grid.z, c.times, f)
-    lon, lat, z = ap.run_oceandrift([rd], c.lon0[:m], c.lat0[:m], c.z0[:m], c.start, c.dt, c.steps, scheme='runge-kutta4', vertical_adv=True)
+    lon, lat, z = ap.run_oceandrift([rd], c.lon0[s], c.lat0[s], c.z0[s], c.start, c.dt, c.steps, scheme='runge-kutta4', vertical_adv=True)
     assert np.array_equal(lon, c.ref['lon'][:m]) and np.array_equal(lat, c.ref['lat'][:m]) and np.array_equal(z, c.ref['z'][:m])

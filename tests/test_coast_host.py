@@ -1,6 +1,8 @@
 """Coastline interaction (tests/coastcases.py) on the host build of the device sources: the drop-in OceanDrift with a gridded
 land_binary_mask reader against runs of the unmodified reference -- surviving elements, deactivated elements in the reference's
 order, their status categories ('stranded', 'seeded_on_land', 'missing_data') and positions."""
+import os
+
 import numpy as np
 import pytest
 
@@ -62,15 +64,10 @@ def test_nearest_sampling_equals_the_reference_interpolator(host_engine):
 @pytest.mark.parametrize('action,scheme,sign,out_every,release', [('stranding', 'runge-kutta4', -1, 1, 3), ('previous', 'euler', -1, 1, 0),
                                                                   ('previous', 'runge-kutta4', 1, 3, 4), ('stranding', 'runge-kutta', 1, 3, 2)])
 def test_coastline_variants_against_the_live_reference(action, scheme, sign, out_every, release, host_engine):
-    """Backward runs, output every third step, release over several steps: the drop-in class beside the unmodified reference
-    (skipped where /root/reference is absent)."""
+    """Backward runs, output every third step, release over several steps: the drop-in class beside the unmodified reference's
+    results on the same runs (recorded in tests/golden/coast_variants_ref.npz)."""
     from datetime import timedelta
     import common
-    from oracle import refrun
-    if not refrun.available():
-        pytest.skip('reference tree not present (GPU box)')
-    refrun.setup()
-    from opendrift.models.oceandrift import OceanDrift as RefOD
     from opendrift_b200.models.oceandrift import OceanDrift
     from opendrift_b200.readers import reader_regular_grid
 
@@ -93,7 +90,15 @@ def test_coastline_variants_against_the_live_reference(action, scheme, sign, out
         o.run(steps=9, time_step=sign * fx.dt, time_step_output=sign * out_every * fx.dt)
         return cc.summary(o)
 
-    r = run(RefOD, lambda lon, lat, z, t, f, name: refrun.make_grid_reader(lon, lat, z, t, f, name=name), logfile='/tmp/od_coast_live.log')
+    def reference():
+        import tempfile
+        from oracle import refrun
+        refrun.setup()
+        from opendrift.models.oceandrift import OceanDrift as RefOD
+        return run(RefOD, lambda lon, lat, z, t, f, name: refrun.make_grid_reader(lon, lat, z, t, f, name=name),
+                   logfile=os.path.join(tempfile.gettempdir(), 'od_coast_live.log'))
+
+    r = common.recorded_reference('coast_variants', '%s_%s_%d_%d_%d' % (action, scheme, sign, out_every, release), reference)
     p = run(OceanDrift, lambda lon, lat, z, t, f, name: reader_regular_grid.Reader(lon, lat, z, t, f, name=name))
     assert list(r['cats']) == list(p['cats']) and np.array_equal(r['id'], p['id'])
     assert np.array_equal(r['d_id'], p['d_id']) and np.array_equal(r['d_status'], p['d_status']) and len(r['d_id']) > 0

@@ -1,6 +1,8 @@
 """Ensemble blocks (tests/enscases.py) on the host build of the device sources: the drop-in OceanDrift against runs of the unmodified
 reference on the same ensemble reader -- member i % n_members per element, also when a second reader serves part of the elements;
 and the reference's own known answer for ReaderBlock with ensemble members (tests/readers/test_interpolation.py:231-259)."""
+import os
+
 import numpy as np
 import pytest
 
@@ -48,14 +50,10 @@ def test_reference_known_answer_for_ensemble_members(host_engine):
                                                                    (2, 'runge-kutta4', 5, 2500, True)])
 def test_ensemble_variants_against_the_live_reference(n_ens, scheme, release, max_age, wind_ens, host_engine):
     """Release over several steps and retirement change an element's rank among the served positions from step to step; a wind
-    reader with its own number of members: the drop-in class beside the unmodified reference (skipped where it is absent)."""
+    reader with its own number of members: the drop-in class beside the unmodified reference's results on the same runs (recorded in
+    tests/golden/ensemble_variants_ref.npz)."""
     from datetime import timedelta
     import common
-    from oracle import refrun
-    if not refrun.available():
-        pytest.skip('reference tree not present (GPU box)')
-    refrun.setup()
-    from opendrift.models.oceandrift import OceanDrift as RefOD
     from opendrift_b200.models.oceandrift import OceanDrift
 
     def run(Model, mk_ens, **kw):
@@ -83,7 +81,16 @@ def test_ensemble_variants_against_the_live_reference(n_ens, scheme, release, ma
         o.run(steps=8, time_step=fx.dt, time_step_output=fx.dt)
         return np.asarray(o.elements.ID), np.asarray(o.elements.lon, dtype=np.float64), np.asarray(o.elements.lat, dtype=np.float64)
 
-    r = run(RefOD, ec.reference_ensemble_reader, logfile='/tmp/ens_live.log')
+    def reference():
+        import tempfile
+        from oracle import refrun
+        refrun.setup()
+        from opendrift.models.oceandrift import OceanDrift as RefOD
+        return dict(zip(('id', 'lon', 'lat'), run(RefOD, ec.reference_ensemble_reader,
+                                                  logfile=os.path.join(tempfile.gettempdir(), 'ens_live.log'))))
+
+    rec = common.recorded_reference('ensemble_variants', '%d_%s_%d_%d_%d' % (n_ens, scheme, release, max_age, wind_ens), reference)
+    r = rec['id'], rec['lon'], rec['lat']
     p = run(OceanDrift, ec.product_ensemble_reader)
     assert np.array_equal(r[0], p[0]) and len(r[0]) > 0
     assert max(common.max_err_deg(p[1], p[2], r[1], r[2])) < 5e-8

@@ -3,7 +3,7 @@
 
   * the oracle pieces that stand in for pyproj (oracle/proj_stere.py, Geod.inv of oracle/geod_karney.py) against mpmath;
   * the NumPy port (oracle/gyre_port.py + oracle/advect_port.py) against the fixtures the UNMODIFIED reference produced
-    (tests/golden/ref_gyre_*.npz, oracle/make_golden.py), bit for bit, and against the live reference when present;
+    (tests/golden/ref_gyre_*.npz, oracle/make_golden.py), bit for bit, and against its recorded runs on random cases;
   * the device code (opendrift_b200/csrc/od_analytic.cuh) compiled for the host against the oracle and the fixtures.
 
 Tolerance.  The box is 2 m x 1 m at (0 E, 0 N): 1e-6 deg (the north-star tolerance) is 0.11 m there, 5 % of the domain,
@@ -11,6 +11,7 @@ so these tests hold 1e-9 deg (1.1e-4 m).  Measured: <= 1.2e-5 m after 60 RK4 ste
 (test_sampler_matches_port); what remains is the ~1e-9 m at which any two implementations of the geodesic agree per
 move (and NumPy's float32 arctan2), amplified by the gyre's chaotic stretching."""
 import ctypes as C
+import os
 from datetime import timedelta
 
 import numpy as np
@@ -99,29 +100,39 @@ def test_port_matches_reference_fixture_bit_for_bit(name):
 
 
 def test_port_matches_live_reference_random_gyre():
-    from oracle import refrun
-    if not refrun.available():
-        pytest.skip('reference tree not present (GPU box)')
-    refrun.setup()
-    from opendrift.readers import reader_double_gyre
-    from opendrift.models.oceandrift import OceanDrift
+    """The port against the unmodified reference's double-gyre runs on random parameters and seeds (recorded in
+    tests/golden/gyre_random_ref.npz: the seeds the reference's reader placed and its final positions)."""
+    from datetime import datetime
     from oracle import advect_port as ap, gyre_port
     rng = np.random.default_rng(5)
     for scheme, dt, n in (('runge-kutta4', 0.07, 300), ('runge-kutta', -0.05, 200), ('euler', 0.2, 1)):
         eps, om, A = rng.uniform(0.05, 0.3), rng.uniform(0.3, 1.0), rng.uniform(0.1, 0.3)
-        dg = reader_double_gyre.Reader(epsilon=eps, omega=om, A=A)
-        lon, lat = dg.xy2lonlat(rng.uniform(-0.02, 2.02, n), rng.uniform(-0.02, 1.02, n))
-        o = OceanDrift(loglevel=50, logfile='/tmp/od_gyre_test.log')
-        o.set_config('environment:fallback:land_binary_mask', 0)
-        o.set_config('general:use_auto_landmask', False)
-        o.set_config('drift:advection_scheme', scheme)
-        o.add_reader(dg)
-        o.seed_elements(lon, lat, time=dg.initial_time)
-        o.run(steps=25, time_step=dt)
-        pr = gyre_port.DoubleGyreReader(dg.initial_time, epsilon=eps, omega=om, A=A)
+        x, y = rng.uniform(-0.02, 2.02, n), rng.uniform(-0.02, 1.02, n)
+
+        def reference():
+            import tempfile
+            from oracle import refrun
+            refrun.setup()
+            from opendrift.readers import reader_double_gyre
+            from opendrift.models.oceandrift import OceanDrift
+            dg = reader_double_gyre.Reader(epsilon=eps, omega=om, A=A)
+            lon, lat = dg.xy2lonlat(x, y)
+            o = OceanDrift(loglevel=50, logfile=os.path.join(tempfile.gettempdir(), 'od_gyre_test.log'))
+            o.set_config('environment:fallback:land_binary_mask', 0)
+            o.set_config('general:use_auto_landmask', False)
+            o.set_config('drift:advection_scheme', scheme)
+            o.add_reader(dg)
+            o.seed_elements(lon, lat, time=dg.initial_time)
+            o.run(steps=25, time_step=dt)
+            return {'seed_lon': lon, 'seed_lat': lat, 'initial_time': dg.initial_time.isoformat(), 'steps': o.steps_calculation,
+                    'lon': o.elements.lon, 'lat': o.elements.lat}
+
+        r = common.recorded_reference('gyre_random', scheme, reference)
+        t0 = datetime.fromisoformat(str(r['initial_time']))
+        pr = gyre_port.DoubleGyreReader(t0, epsilon=eps, omega=om, A=A)
         # (the reference runs int(duration / time_step) steps: 24 for 25 * 0.07 s)
-        pl, pa, _ = ap.run_oceandrift([pr], lon, lat, np.zeros(n), dg.initial_time, dt, o.steps_calculation, scheme=scheme)
-        assert np.array_equal(pl, o.elements.lon) and np.array_equal(pa, o.elements.lat), scheme
+        pl, pa, _ = ap.run_oceandrift([pr], r['seed_lon'], r['seed_lat'], np.zeros(n), t0, dt, int(r['steps']), scheme=scheme)
+        assert np.array_equal(pl, r['lon']) and np.array_equal(pa, r['lat']), scheme
 
 
 # ---- the device code, compiled for the host ----------------------------------------------------------------------------
@@ -303,11 +314,10 @@ def test_reader_and_environment_calls_on_host_engine():
 @pytest.mark.parametrize('proj4', gc.ASPECTS)
 def test_other_projection_aspects_whole_run(proj4):
     """The double gyre placed on oblique and polar stereographic planes and across the dateline: host-compiled device
-    code against the port, and the port against the live reference when it is present.  (At these latitudes the float32
-    seed arrays of the reference quantise the 2 m box to a few distinct positions -- parity is what is checked, not
-    oceanography.  Readers north of 89 deg are discarded by the reference's simulation extent,
+    code against the port, and the port against the unmodified reference's results (tests/golden/gyre_aspects_ref.npz).
+    (At these latitudes the float32 seed arrays of the reference quantise the 2 m box to a few distinct positions -- parity
+    is what is checked, not oceanography.  Readers north of 89 deg are discarded by the reference's simulation extent,
     basemodel/__init__.py:2026-2034, hence the offsets.)"""
-    from oracle import refrun
     fx = gc.AspectCase(proj4)
     sx, sy = fx.plane.forward(fx.seed_lon.astype(np.float32).astype(np.float64), fx.seed_lat.astype(np.float32).astype(np.float64))
     px, py = fx.plane.forward(fx.lon, fx.lat)
@@ -318,20 +328,26 @@ def test_other_projection_aspects_whole_run(proj4):
     o, _ = _model(fx, HostEngine())                              # the drop-in classes on the host build
     o.run(steps=fx.steps, time_step=fx.dt)
     assert np.array_equal(np.asarray(o.elements.lon), hl) and np.array_equal(np.asarray(o.elements.lat), ha)
-    if refrun.available():
+
+    def reference():
+        import tempfile
+        from oracle import refrun
         refrun.setup()
         from opendrift.readers import reader_double_gyre
         from opendrift.models.oceandrift import OceanDrift
         dg = reader_double_gyre.Reader(initial_time=fx.t0, proj4=proj4, **fx.par)
-        o = OceanDrift(loglevel=50, logfile='/tmp/od_gyre_test.log')
+        o = OceanDrift(loglevel=50, logfile=os.path.join(tempfile.gettempdir(), 'od_gyre_test.log'))
         o.set_config('environment:fallback:land_binary_mask', 0)
         o.set_config('general:use_auto_landmask', False)
         o.set_config('drift:advection_scheme', fx.scheme)
         o.add_reader(dg)
         o.seed_elements(fx.seed_lon, fx.seed_lat, time=fx.t0)
         o.run(steps=fx.steps, time_step=fx.dt)
-        assert o.steps_calculation == fx.steps
-        assert np.array_equal(fx.lon, o.elements.lon) and np.array_equal(fx.lat, o.elements.lat)
+        return {'steps': o.steps_calculation, 'lon': o.elements.lon, 'lat': o.elements.lat}
+
+    r = common.recorded_reference('gyre_aspects', 'aspect%d' % gc.ASPECTS.index(proj4), reference)
+    assert int(r['steps']) == fx.steps
+    assert np.array_equal(fx.lon, r['lon']) and np.array_equal(fx.lat, r['lat'])
 
 
 def test_bench_extra_measurement_runs_on_host_engine():

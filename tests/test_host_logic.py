@@ -242,26 +242,38 @@ def test_field_group_prefetches_the_next_slab_on_the_copy_stream():
 def test_config_keys_match_the_reference_model_classes():
     """set_config / get_config of a script written for the reference must not raise here: OceanDrift and Leeway expose the
     reference's configuration keys (plus gpu:*), with its defaults except general:coastline_action (no landmask on the GPU
-    path: 'none')."""
-    from oracle import refrun
-    if not refrun.available():
-        pytest.skip('reference tree not present (GPU box)')
-    refrun.setup()
-    import opendrift.models.oceandrift as ro
-    import opendrift.models.leeway as rl
+    path: 'none').  The reference's keys and defaults are recorded in tests/golden/config_keys_ref.npz."""
+    import json
+    import common
     import opendrift_b200.models.oceandrift as po
     import opendrift_b200.models.leeway as pl
 
+    def plain(v):                       # a default as JSON holds it (the recorded form)
+        return json.loads(json.dumps(v, default=repr))
+
+    def reference():
+        import os
+        import tempfile
+        from oracle import refrun
+        refrun.setup()
+        import opendrift.models.oceandrift as ro
+        import opendrift.models.leeway as rl
+        log = os.path.join(tempfile.gettempdir(), 'od_cfg_test.log')
+        return {R.__name__: json.dumps({k: plain(c.get('default')) for k, c in R(loglevel=50, logfile=log)._config.items()})
+                for R in (ro.OceanDrift, rl.Leeway)}
+
+    rec = common.recorded_reference('config_keys', 'defaults', reference)
+
     class NoEngine:
         pass
-    for R, P, extra in ((ro.OceanDrift, po.OceanDrift, set()), (rl.Leeway, pl.Leeway, {'general:seafloor_action', 'seed:seafloor'})):
-        r, p = R(loglevel=50, logfile='/tmp/od_cfg_test.log'), P(loglevel=50, engine=NoEngine())
-        rk, pk = set(r._config), set(p._config)
+    for P, extra in ((po.OceanDrift, set()), (pl.Leeway, {'general:seafloor_action', 'seed:seafloor'})):
+        r, p = json.loads(str(rec[P.__name__])), P(loglevel=50, engine=NoEngine())
+        rk, pk = set(r), set(p._config)
         assert rk - pk == set(), sorted(rk - pk)
         assert {k for k in pk - rk if not k.startswith('gpu:')} == extra
         for k in rk & pk:
             if k != 'general:coastline_action':
-                assert r._config[k].get('default') == p._config[k].get('default'), k
+                assert r[k] == plain(p._config[k].get('default')), k
     o = po.OceanDrift(loglevel=50, engine=NoEngine())
     o.set_config('general:simulation_name', 'my run')
     o.set_config('seed:z', -5)

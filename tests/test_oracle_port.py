@@ -1,6 +1,6 @@
 """The NumPy port (oracle/advect_port.py) is pinned to the UNMODIFIED reference: bit-identical final
-positions on every committed fixture (tests/golden/ref_*.npz, written by oracle/make_golden.py from a
-live run of /root/reference), and - when the reference tree is present - on a fresh random case."""
+positions on every committed fixture (tests/golden/ref_*.npz, written by oracle/make_golden.py from live runs of
+the reference) and on the reference's recorded results of fresh random cases."""
 import numpy as np
 import pytest
 
@@ -30,9 +30,8 @@ def test_leeway_port_matches_reference_fixture(name):
 
 
 def test_port_matches_live_reference():
-    from oracle import refrun
-    if not refrun.available():
-        pytest.skip('reference tree not present (GPU box)')
+    """The port against the unmodified reference on a fresh random case (its final positions recorded in
+    tests/golden/port_live_ref.npz)."""
     from oracle import advect_port as ap
     from opendrift_b200 import synthetic as syn
     g = syn.GridSpec(nx=30, ny=28, nz=6, lon0=1.0, dlon=0.07, lat0=57.0, dlat=0.04, dz=15.0)
@@ -43,11 +42,17 @@ def test_port_matches_live_reference():
     lon = rng.uniform(1.3, 2.8, 400).astype(np.float32)
     lat = rng.uniform(57.2, 58.0, 400).astype(np.float32)
     z = rng.uniform(-80, 0, 400).astype(np.float32)
-    o = refrun.run_oceandrift([refrun.make_grid_reader(g.lon, g.lat, g.z, times, fields)], lon, lat, z, syn.T0,
-                              900, 5, config={'drift:advection_scheme': 'runge-kutta4',
-                                              'drift:vertical_advection': False})
+
+    def reference():
+        from oracle import refrun
+        o = refrun.run_oceandrift([refrun.make_grid_reader(g.lon, g.lat, g.z, times, fields)], lon, lat, z, syn.T0,
+                                  900, 5, config={'drift:advection_scheme': 'runge-kutta4',
+                                                  'drift:vertical_advection': False})
+        return {'lon': o.elements.lon, 'lat': o.elements.lat}
+
+    r = common.recorded_reference('port_live', 'rk4', reference)
     pl, pa, _ = ap.run_oceandrift([ap.GridReader(g.lon, g.lat, g.z, times, fields)], lon, lat, z, syn.T0, 900, 5)
-    assert np.array_equal(pl, o.elements.lon) and np.array_equal(pa, o.elements.lat)
+    assert np.array_equal(pl, r['lon']) and np.array_equal(pa, r['lat'])
 
 
 def _run_reference(fx):
@@ -77,19 +82,22 @@ def _run_reference(fx):
 @pytest.mark.parametrize('family,seed', [('basic', 0), ('basic', 3), ('basic', 4), ('basic', 7), ('options', 3), ('options', 6),
                                          ('options', 21), ('readers', 1), ('readers', 4), ('readers', 9), ('wdf', 1), ('wdf', 2)])
 def test_port_matches_live_reference_on_random_scenarios(family, seed):
-    """The port against the UNMODIFIED reference (this container only) on the randomised scenarios that the device math is
-    checked with: descending axes, periodic and global grids, own-grid vertical velocity, truncation, land holes, node and
-    level particles, float32 drift-factor arrays, backward runs.  Bit for bit."""
-    from oracle import refrun
-    if not refrun.available():
-        pytest.skip('reference tree not present (GPU box)')
+    """The port against the UNMODIFIED reference on the randomised scenarios that the device math is checked with: descending
+    axes, periodic and global grids, own-grid vertical velocity, truncation, land holes, node and level particles, float32
+    drift-factor arrays, backward runs.  Bit for bit, against the reference's final states recorded in
+    tests/golden/port_random_ref.npz."""
     import test_hostmath as th
     fx = {'basic': th._random_scenario, 'options': th._random_options_scenario, 'readers': th._random_readers_scenario,
           'wdf': th._random_wdf_scenario}[family](seed)
     if fx is None or fx.meta.get('noise'):
         pytest.skip('scenario not applicable for this seed')
-    o = _run_reference(fx)
-    assert len(o.elements.lon) == fx.n
+
+    def reference():
+        o = _run_reference(fx)
+        return {'lon': o.elements.lon, 'lat': o.elements.lat, 'z': o.elements.z}
+
+    r = common.recorded_reference('port_random', '%s%d' % (family, seed), reference)
+    assert len(r['lon']) == fx.n
     pl, pa, pz = common.run_port(fx)
-    assert np.array_equal(pl, np.asarray(o.elements.lon)) and np.array_equal(pa, np.asarray(o.elements.lat))
-    assert np.array_equal(np.asarray(pz, dtype=np.float64), np.asarray(o.elements.z, dtype=np.float64))
+    assert np.array_equal(pl, r['lon']) and np.array_equal(pa, r['lat'])
+    assert np.array_equal(np.asarray(pz, dtype=np.float64), np.asarray(r['z'], dtype=np.float64))

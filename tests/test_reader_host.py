@@ -11,15 +11,12 @@ def test_reader_output_equals_the_reference_reader_bit_for_bit():
 def test_projected_reader_output_beside_the_live_reference():
     """get_variables_interpolated of readers on conic / stereographic / Mercator planes, with and without the rotation to east /
     north (rotate_to_proj): unrotated values bit-equal, rotated ones to 1e-9 (the rotation angle comes from a differently organised
-    inverse geodesic) and float64 like the reference's."""
+    inverse geodesic) and float64 like the reference's.  The reference reader's output is recorded in
+    tests/golden/reader_proj_ref.npz."""
     import numpy as np
-    import pytest
     from datetime import timedelta
+    import common
     import projcases as pc
-    from oracle import refrun
-    if not refrun.available():
-        pytest.skip('reference tree not present (GPU box)')
-    refrun.setup()
     from opendrift_b200.readers import reader_regular_grid
     eng = HostEngine()
     for case in ('lcc_wgs84_rk4_3d_w', 'stere_wgs84_polar_rk4_3d_w', 'merc_sphere_mixing', 'lcc_sphere_rk2_wind'):
@@ -29,14 +26,23 @@ def test_projected_reader_output_beside_the_live_reference():
         f = {k: v for k, v in fields[nm].items() if 'velocity' in k and 'upward' not in k}
         rp = reader_regular_grid.Reader(xs, ys, zs if three_d else None, times, f, name=nm, proj4=c['proj4'])
         rp.bind(eng)
-        rr = refrun.make_grid_reader(xs, ys, zs if three_d else None, times, f, name=nm, proj4=c['proj4'])
         t = times[0] + timedelta(seconds=1000)
         lon, lat, z = lon0.astype(np.float64), lat0.astype(np.float64), z0.astype(np.float64)
-        for rot in (None, '+proj=latlong'):
+        rots = {'plain': None, 'rotated': '+proj=latlong'}
+
+        def reference():
+            from oracle import refrun
+            rr = refrun.make_grid_reader(xs, ys, zs if three_d else None, times, f, name=nm, proj4=c['proj4'])
+            out = {}
+            for tag, rot in rots.items():
+                b, _ = rr.get_variables_interpolated(list(f), time=t, lon=lon, lat=lat, z=z, rotate_to_proj=rot)
+                out.update({'%s_%s' % (tag, k): np.ma.filled(np.ma.masked_invalid(b[k]), np.nan) for k in f})
+            return out
+        b = common.recorded_reference('reader_proj', case, reference)
+        for tag, rot in rots.items():
             a, _ = rp.get_variables_interpolated(list(f), time=t, lon=lon, lat=lat, z=z, rotate_to_proj=rot)
-            b, _ = rr.get_variables_interpolated(list(f), time=t, lon=lon, lat=lat, z=z, rotate_to_proj=rot)
             for k in f:
-                x, y = np.ma.filled(np.ma.masked_invalid(a[k]), np.nan), np.ma.filled(np.ma.masked_invalid(b[k]), np.nan)
+                x, y = np.ma.filled(np.ma.masked_invalid(a[k]), np.nan), b['%s_%s' % (tag, k)]
                 assert x.dtype == y.dtype, (case, rot, k, x.dtype, y.dtype)
                 if rot is None:
                     assert np.array_equal(x, y, equal_nan=True)
@@ -92,15 +98,11 @@ def test_check_arguments_as_reference_style_readers_call_it():
 
 def test_sub_block_reader_queries_beside_the_live_reference():
     """Reader-level queries on readers that hand out sub-blocks: the block around the positions of the call, the block's own index
-    geometry -- bit-equal to the reference's StructuredReader on a reader of the same kind (2-D float32, 3-D float64)."""
+    geometry -- bit-equal to the reference's StructuredReader on a reader of the same kind (2-D float32, 3-D float64), whose output
+    is recorded in tests/golden/reader_subblock_ref.npz."""
     import numpy as np
-    import pytest
     from datetime import timedelta
     import common
-    from oracle import refrun
-    if not refrun.available():
-        pytest.skip('reference tree not present (GPU box)')
-    refrun.setup()
     from opendrift_b200.readers import reader_regular_grid
     for fxn in ('rk4_2d', 'rk4_3d'):
         fx = common.Fixture(fxn)
@@ -109,12 +111,18 @@ def test_sub_block_reader_queries_beside_the_live_reference():
         for sl in (slice(0, 200), slice(200, 230), slice(0, 1500)):
             lon, lat = fx.lon0[sl].astype(np.float64), fx.lat0[sl].astype(np.float64)
             z = np.zeros(len(lon)) if fx.grid_z is None else fx.z0[sl].astype(np.float64)
-            rr = refrun.make_grid_reader(fx.grid_lon, fx.grid_lat, fx.grid_z, fx.times, fields, name='r', subblocks=True)
+
+            def reference():
+                from oracle import refrun
+                rr = refrun.make_grid_reader(fx.grid_lon, fx.grid_lat, fx.grid_z, fx.times, fields, name='r', subblocks=True)
+                rr.buffer = 3
+                a, _ = rr.get_variables_interpolated(list(fields), time=t, lon=lon, lat=lat, z=z)
+                return {k: np.ma.filled(np.ma.masked_invalid(a[k]), np.nan) for k in fields}
+            a = common.recorded_reference('reader_subblock', '%s_%d_%d' % (fxn, sl.start, sl.stop), reference)
             rp = reader_regular_grid.Reader(fx.grid_lon, fx.grid_lat, fx.grid_z, fx.times, fields, name='r', subblocks=True)
-            rr.buffer = rp.buffer = 3
+            rp.buffer = 3
             rp.bind(HostEngine())
-            a, _ = rr.get_variables_interpolated(list(fields), time=t, lon=lon, lat=lat, z=z)
             b, _ = rp.get_variables_interpolated(list(fields), time=t, lon=lon, lat=lat, z=z)
             for k in fields:
-                x, y = np.ma.filled(np.ma.masked_invalid(a[k]), np.nan), np.ma.filled(np.ma.masked_invalid(b[k]), np.nan)
+                x, y = a[k], np.ma.filled(np.ma.masked_invalid(b[k]), np.nan)
                 assert x.dtype == y.dtype and np.array_equal(x, y, equal_nan=True), (fxn, sl, k)
